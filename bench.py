@@ -60,6 +60,9 @@ def parse():
                     help="reads of the C3-shaped polishing run (0 = skip)")
     ap.add_argument("--c5-reads", type=int, default=30_000,
                     help="HiFi reads of the C5-shaped run: stage 1 + identity filter (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the stage-1 result of the last timed step to DIR/<name>.npy "
+                         "(a fixed, seeded sample of the reads; at most 64 MB)")
     return ap.parse_args()
 
 
@@ -188,6 +191,44 @@ def same_result(x, y):
                for k in ("overlaps", "ovl_off", "pile"))
 
 
+DUMP_BYTES = 64 << 20
+DUMP_MAX_READS = 4096
+
+
+def gather_ranges(values, off, ids):
+    """values[off[i]:off[i + 1]] of every read i in ids, concatenated, and their lengths."""
+    import numpy as np
+    o = off.astype(np.int64)
+    cnt = o[ids + 1] - o[ids]
+    idx = np.repeat(o[ids], cnt) + (np.arange(int(cnt.sum())) - np.repeat(np.cumsum(cnt) - cnt, cnt))
+    return values[idx], cnt
+
+
+def dump_outputs(path, res, budget, suffix=""):
+    """The stage-1 result a caller receives (kept overlaps and pile of every read, the
+    number of mapped overlaps) as float .npy files, for a fixed, seeded sample of the
+    reads that fits `budget` bytes. float64 holds the uint32/uint64 fields exactly,
+    float32 the uint16 pile bins. Files: read_ids, overlaps (one row of 8 fields per
+    kept overlap of the sampled reads, in read order), overlaps_per_read, pile (the
+    bins of the sampled reads), bins_per_read, num_mapped."""
+    import numpy as np
+    n = len(res["ovl_off"]) - 1
+    per_read = (8 * 8 * np.diff(res["ovl_off"].astype(np.int64))
+                + 4 * np.diff(res["pile_off"].astype(np.int64)) + 3 * 8)
+    order = np.random.default_rng(SEED).permutation(n)
+    fits = int(np.searchsorted(np.cumsum(per_read[order]), budget - 4096, side="right"))  # npy headers
+    ids = np.sort(order[:min(fits, DUMP_MAX_READS)])
+    ovl, n_ovl = gather_ranges(np.asarray(res["overlaps"]).reshape(-1, 8), res["ovl_off"], ids)
+    pile, n_bins = gather_ranges(np.asarray(res["pile"]), res["pile_off"], ids)
+    out = {"read_ids": ids.astype(np.float64), "overlaps": ovl.astype(np.float64),
+           "overlaps_per_read": n_ovl.astype(np.float64), "pile": pile.astype(np.float32),
+           "bins_per_read": n_bins.astype(np.float64),
+           "num_mapped": np.array([res["num_mapped"]], dtype=np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), arr)
+
+
 def share_of(res, rank, world):
     """The slice of a complete stage-1 result that rank `rank` owns (reads rank,
     rank + world, ...), in the layout of DistEngine's per-rank result."""
@@ -196,11 +237,7 @@ def share_of(res, rank, world):
     ids = np.arange(rank, n, world)
     out = {}
     for key, off in (("overlaps", "ovl_off"), ("pile", "pile_off")):
-        o = res[off].astype(np.int64)
-        cnt = (o[ids + 1] - o[ids])
-        idx = np.repeat(o[ids], cnt) + (np.arange(int(cnt.sum())) -
-                                         np.repeat(np.cumsum(cnt) - cnt, cnt))
-        out[key] = res[key][idx]
+        out[key], cnt = gather_ranges(res[key], res[off], ids)
         out[off] = np.concatenate([[0], np.cumsum(cnt)]).astype(np.uint64)
     return out
 
@@ -328,6 +365,11 @@ def main_ours(a):
     launches_step = st["kernel_launches"]
     n_mapped = st["overlaps"]
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs:        # the results of the LAST timed step (this rank's share)
+        dump_outputs(a.dump_outputs,
+                     distributed.CudaSteps(eng, f"cuda:{local}").stage1_results() if world > 1
+                     else eng.stage1_results(),
+                     DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
 
     for _ in range(1):
         step_e2e()

@@ -200,8 +200,10 @@ class Engine:
         self._check(self.lib.rvn_find_overlaps_and_create_piles(
             self.h, float(freq), max_overlaps, int(use_minhash), index_batch_bases,
             query_batch_bases))
-        if not fetch:
-            return None
+        return self.stage1_results() if fetch else None
+
+    def stage1_results(self):
+        """Host copies of the last find_overlaps_and_create_piles call's results."""
         o, off, p, poff, nm = OVLP(), U64P(), U16P(), U64P(), C.c_uint64(0)
         self._check(self.lib.rvn_stage1_results(self.h, C.byref(o), C.byref(off),
                                                 C.byref(p), C.byref(poff),

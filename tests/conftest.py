@@ -21,14 +21,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def reference():
-    import oracle_lib
-    if not oracle_lib.Reference.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return oracle_lib.Reference()
-
-
-@pytest.fixture(scope="session")
 def lambda_reads():
     from raven_b200 import seqio
     return seqio.ReadSet.load(os.path.join(ROOT, "tests", "golden", "lambda_reads.npz"))

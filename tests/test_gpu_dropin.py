@@ -2,6 +2,7 @@
 running on the B200 engine through the ram::MinimizerEngine facade, and our
 batched FindOverlapsAndCreatePiles replacement with the reference signature -
 both against the CPU oracle, bit exact."""
+import json
 import os
 import struct
 import subprocess
@@ -15,6 +16,15 @@ pytestmark = pytest.mark.gpu
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 BIN = os.path.join(HERE, "cpp", "_build", "dropin_test")
+REF_META = json.load(open(os.path.join(HERE, "golden", "reference_golden.json")))
+REF_GOLD = np.load(os.path.join(HERE, "golden", "reference_golden.npz"))
+
+
+def reference_assembly():
+    """RavenTest.Assemble's polished unitigs from the reference's own sources over the
+    CPU oracle (stored by tests/golden/make_reference_golden.py): names and sequences."""
+    names = REF_META["assemble_rounds2_names"]
+    return names, [REF_GOLD[f"assemble_rounds2_unitig{i}"].tobytes() for i in range(len(names))]
 
 
 def write_vec(f, a):
@@ -29,7 +39,7 @@ def read_vec(f, dt):
 
 def run_dropin(tmp_path, rs, k, w, freq, kmax, minhash):
     if not os.path.exists(BIN):
-        pytest.skip("tests/cpp/_build/dropin_test not built (needs /root/reference at build time)")
+        pytest.skip("tests/cpp/_build/dropin_test not built (needs the reference's sources at build time)")
     inp, out = str(tmp_path / "reads.bin"), str(tmp_path / "out.bin")
     with open(inp, "wb") as f:
         write_vec(f, rs.words.astype(np.uint64))
@@ -66,12 +76,11 @@ def test_dropin_synthetic_small_kmax(tmp_path, oracle):
             assert np.array_equal(got[key], want[key]), key
 
 
-def test_full_pipeline_on_b200_equals_oracle_pipeline(tmp_path, oracle, reference, lambda_reads):
+def test_full_pipeline_on_b200_equals_oracle_pipeline(tmp_path, oracle, lambda_reads):
     """RavenTest.Assemble with the reference's own sources on the B200 facades
     (ram::MinimizerEngine, racon::Polisher incl. GPU POA) == the same sources over
     the CPU oracle: identical polished unitig, and the reference's golden value:
     1137 edits to NC_001416 (RavenTest/src/raven_test.cpp:66)."""
-    import oracle_lib
     from raven_b200 import seqio
     binary = os.path.join(HERE, "cpp", "_build", "assemble_test")
     if not os.path.exists(binary):
@@ -87,7 +96,7 @@ def test_full_pipeline_on_b200_equals_oracle_pipeline(tmp_path, oracle, referenc
                    timeout=900)
     lines = open(out).read().split("\n")
     names, seqs = lines[0:-1:2], [s.encode() for s in lines[1::2]]
-    want_names, want_seqs = oracle_lib.ref_assemble(reference, lambda_reads, True, 2, 8)
+    want_names, want_seqs = reference_assembly()
     assert names == want_names
     assert seqs == want_seqs
     genome = seqio.ReadSet.load(os.path.join(HERE, "golden", "lambda_genome.npz")).ascii(0)
@@ -125,7 +134,7 @@ def test_stage2_and_identity_filter_batched_equals_reference(tmp_path, lambda_re
         assert a[0].size == 0                  # ... but no pair of 10 % error reads is 90 % identical
 
 
-def test_reference_cli_runs_on_b200(tmp_path, oracle, reference, lambda_reads):
+def test_reference_cli_runs_on_b200(tmp_path, oracle, lambda_reads):
     """The reference's own executable (RavenExe/src/main.cc + all of RavenLib,
     unmodified; tests/cpp/Makefile `_build/raven`) over the drop-in dependencies:
     FASTQ.gz in (bioparser), overlap + layout + 2 polishing rounds on the B200,
@@ -133,7 +142,6 @@ def test_reference_cli_runs_on_b200(tmp_path, oracle, reference, lambda_reads):
     and its golden value; then `--resume` from the checkpoint (cereal) gives the
     same answer (RavenTest.Checkpoints, raven_test.cpp:69-95)."""
     import gzip
-    import oracle_lib
     from raven_b200 import seqio
     binary = os.path.join(HERE, "cpp", "_build", "raven")
     if not os.path.exists(binary):
@@ -151,7 +159,7 @@ def test_reference_cli_runs_on_b200(tmp_path, oracle, reference, lambda_reads):
                                     stderr=subprocess.DEVNULL, timeout=900).stdout
     out = run("-p", "2", "-F", "graph.gfa").decode().split("\n")
     names, seqs = out[0:-1:2], [s.encode() for s in out[1::2]]
-    want_names, want_seqs = oracle_lib.ref_assemble(reference, rs, True, 2, 8)
+    want_names, want_seqs = reference_assembly()
     assert [n[1:] for n in names] == want_names
     assert seqs == want_seqs
     genome = seqio.ReadSet.load(os.path.join(HERE, "golden", "lambda_genome.npz")).ascii(0)

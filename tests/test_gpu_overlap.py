@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+import reference_inputs as inputs
 from raven_b200 import seqio, synth
 
 pytestmark = pytest.mark.gpu
@@ -13,6 +14,8 @@ pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 META = json.load(open(os.path.join(HERE, "golden", "lambda_golden.json")))
 GOLD = np.load(os.path.join(HERE, "golden", "lambda_golden.npz"))
+REF_META = json.load(open(os.path.join(HERE, "golden", "reference_golden.json")))
+REF_GOLD = np.load(os.path.join(HERE, "golden", "reference_golden.npz"))
 
 
 def edge_reads():
@@ -330,21 +333,20 @@ def test_stage1_probe_path_without_self_join(gpu_engine, oracle, lambda_reads):
 def test_stage1_pile_regions_equal_reference(gpu_engine, lambda_reads):
     """rvn_stage1_pile_regions (Pile::FindValidRegion(4) + FindMedian on the piles stage 1
     left on the device, construct.cc:134-139) against the reference's own pile.cc compiled
-    in place (oracle/_ref): begin, end, median, invalid of every pile - the lambda reads,
-    a deep synthetic set, other coverages; and the state check."""
-    import oracle_lib
-    if not oracle_lib.Reference.available():
-        pytest.skip("oracle/_ref not built")
-    ref = oracle_lib.Reference()
-    for rs in (lambda_reads, synth.make_reads(40_000, 300, 5000, seed=14)):
+    in place (its results on the reference's stage-1 piles stored): begin, end, median,
+    invalid of every pile - the lambda reads, a deep synthetic set, other coverages; and
+    the state check."""
+    import hashlib
+    for name, rs in (("lambda", lambda_reads), ("synthetic", inputs.region_reads())):
         gpu_engine.configure(15, 5)
         gpu_engine.upload(rs)
         res = gpu_engine.find_overlaps_and_create_piles(0.001, 32, False)
-        for cov in (4, 1, 9, 30):
+        assert (hashlib.sha256(np.ascontiguousarray(res["pile"]).tobytes()).hexdigest()
+                == REF_META[f"regions_{name}_pile_sha256"])
+        for cov in inputs.REGION_COVERAGES:
             got = gpu_engine.stage1_pile_regions(cov)
-            want = oracle_lib.ref_pile_trim(ref, res["pile"], res["pile_off"], cov)
             for k in ("invalid", "begin", "end", "median"):
-                assert np.array_equal(got[k], want[k]), (cov, k)
+                assert np.array_equal(got[k], REF_GOLD[f"regions_{name}_cov{cov}_{k}"]), (cov, k)
         assert (got["invalid"] == 0).any() or rs is lambda_reads
     assert (gpu_engine.stage1_pile_regions(4)["invalid"] == 0).sum() > 100
     gpu_engine.upload(rs)
@@ -420,8 +422,7 @@ def test_stage1_hifi_params(gpu_engine, oracle):
 
 def test_kmer_complexity(gpu_engine, oracle):
     """Pile::AddKmers' low-complexity rule on the positions Map reports as filtered."""
-    from test_oracle import _lowcomplexity_reads
-    rs = _lowcomplexity_reads()
+    rs = inputs.lowcomplexity_reads()
     gpu_engine.configure(15, 5)
     gpu_engine.upload(rs)
     idx, pos = [], []
