@@ -30,6 +30,7 @@
 #include <cstring>
 
 #include "engine.cuh"
+#include "seed.cuh"
 
 namespace rvn {
 
@@ -120,72 +121,6 @@ __global__ void GatherBoundaries(const uint64_t* __restrict__ src, uint64_t stri
 // ---------------------------------------------------------------------------
 // seed lookup of received queries, hits written into per-destination runs
 // ---------------------------------------------------------------------------
-struct IndexView2 {
-  ValView val;
-  const uint64_t* org;
-  const uint32_t* bucket;
-  uint64_t n;
-  int shift;
-  uint32_t occurrence;
-  uint64_t limit;  // values beyond it are not indexed (tiered build)
-};
-
-__device__ __forceinline__ void Lookup2(const IndexView2& ix, uint64_t v, uint32_t* first,
-                                        uint32_t* count) {
-  if (v > ix.limit) {
-    *first = 0;
-    *count = 0;
-    return;
-  }
-  const uint64_t b = v >> ix.shift;
-  uint32_t lo = ix.bucket[b], hi = ix.bucket[b + 1];
-  while (hi - lo > 8) {
-    const uint32_t mid = lo + (hi - lo) / 2;
-    if (ix.val[mid] < v) lo = mid + 1; else hi = mid;
-  }
-  const uint32_t end = ix.bucket[b + 1];
-  while (lo < end && ix.val[lo] < v) ++lo;
-  if (lo >= end || ix.val[lo] != v) {
-    *first = 0;
-    *count = 0;
-    return;
-  }
-  *first = lo;
-  if (ix.occurrence != 0xFFFFFFFFu && static_cast<uint64_t>(lo) + ix.occurrence < ix.n &&
-      ix.val[static_cast<uint64_t>(lo) + ix.occurrence] == v) {
-    *count = ix.occurrence + 1;
-    return;
-  }
-  uint32_t n = 1;
-  while (static_cast<uint64_t>(lo) + n < ix.n && ix.val[lo + n] == v) ++n;
-  *count = n;
-}
-
-__device__ __forceinline__ bool Keep2(uint32_t lhs_id, uint64_t origin, bool ae, bool as) {
-  const uint32_t rhs_id = static_cast<uint32_t>(origin >> 32);
-  if (ae && lhs_id == rhs_id) return false;
-  if (as && lhs_id > rhs_id) return false;
-  return true;
-}
-
-__global__ void __launch_bounds__(kThreads)
-ProbeOwned(IndexView2 ix, const uint64_t* __restrict__ q_val,
-           const uint64_t* __restrict__ q_org, uint64_t n_q, bool ae, bool as,
-           uint32_t* __restrict__ cnt, uint32_t* __restrict__ first) {
-  const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
-  if (i >= n_q) return;
-  const uint64_t v = q_val[i];
-  const uint32_t lhs_id = static_cast<uint32_t>(q_org[i] >> 32);
-  uint32_t f, n;
-  Lookup2(ix, v, &f, &n);
-  uint32_t kept = 0;
-  if (n <= ix.occurrence) {
-    for (uint32_t j = 0; j < n; ++j) kept += Keep2(lhs_id, ix.org[f + j], ae, as);
-  }
-  cnt[i] = kept;
-  first[i] = f;
-}
-
 // the received query records are sorted by read id:
 // start[r] = first query record of a read >= r, for r in [0, n_reads]
 __global__ void QueryReadStarts(const uint64_t* __restrict__ q_org, uint64_t n_q,
@@ -217,7 +152,7 @@ __global__ void ReadHitTotals(const uint64_t* __restrict__ start,
 }
 
 __global__ void __launch_bounds__(kThreads)
-ExpandOwned(IndexView2 ix, const uint64_t* __restrict__ q_val,
+ExpandOwned(IndexView ix, const uint64_t* __restrict__ q_val,
             const uint64_t* __restrict__ q_org, uint64_t n_q, bool ae, bool as,
             const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ first,
             const uint64_t* __restrict__ hit_off, const uint64_t* __restrict__ start,
@@ -235,110 +170,38 @@ ExpandOwned(IndexView2 ix, const uint64_t* __restrict__ q_val,
   uint32_t left = cnt[i];
   if (left == 0) return;
   const uint64_t v = q_val[i];
-  const uint64_t lhs_pos = static_cast<uint32_t>(lo) >> 1;
-  uint64_t dst = read_base[Slot(lhs_id, parts, per_part)] + (hit_off[i] - hit_off[start[lhs_id]]);
-  for (uint64_t j = first[i]; left > 0 && j < ix.n && ix.val[j] == v; ++j) {
-    const uint64_t o = ix.org[j];
-    if (!Keep2(lhs_id, o, ae, as)) continue;
-    const uint64_t rhs_id = o >> 32;
-    const uint64_t strand = (lo & 1) == (o & 1);
-    const uint64_t rhs_pos = static_cast<uint32_t>(o) >> 1;
-    const uint64_t diagonal =
-        !strand ? rhs_pos + lhs_pos : rhs_pos - lhs_pos + (3ULL << 30);
-    h_grp[dst] = (((rhs_id << 1) | strand) << 32) | diagonal;
-    h_pos[dst] = (lhs_pos << 32) | rhs_pos;
-    h_lhs[dst] = lhs_id;
-    ++dst;
-    --left;
-  }
+  const uint64_t dst =
+      read_base[Slot(lhs_id, parts, per_part)] + (hit_off[i] - hit_off[start[lhs_id]]);
+  // (h_lhs is always given: without the hint the shared loop tests it per hit, and its
+  //  postings are no longer loaded through the read-only path)
+  __builtin_assume(h_lhs != nullptr);
+  ExpandQuery(ix, v, lo, first[i], left, ae, as, dst, h_grp, h_pos, h_lhs);
 }
 
-// the same two steps for the stage-1 flags (avoid_equal && avoid_symmetric): the
-// kept postings are a suffix of the run (see map.cu: ProbeSuffixKernel), the
-// expansion is done by whole warps with coalesced stores
+// the kept postings are contiguous (seed.cuh): whole warps, coalesced loads
 __global__ void __launch_bounds__(kThreads)
-ProbeOwnedSuffix(IndexView2 ix, const uint64_t* __restrict__ q_val,
-                 const uint64_t* __restrict__ q_org, uint64_t n_q,
-                 uint32_t* __restrict__ cnt, uint32_t* __restrict__ first) {
-  const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
-  if (i >= n_q) return;
-  const uint64_t v = q_val[i];
-  const uint32_t lhs_id = static_cast<uint32_t>(q_org[i] >> 32);
-  uint32_t f, n;
-  Lookup2(ix, v, &f, &n);
-  uint32_t kept = 0, fk = f;
-  if (n <= ix.occurrence && n > 0) {
-    uint32_t lo = f, hi = f + n;  // first posting with rhs_id > lhs_id
-    while (lo < hi) {
-      const uint32_t mid = lo + (hi - lo) / 2;
-      if (static_cast<uint32_t>(ix.org[mid] >> 32) <= lhs_id) lo = mid + 1; else hi = mid;
-    }
-    fk = lo;
-    kept = f + n - fk;
-  }
-  cnt[i] = kept;
-  first[i] = fk;
-}
-
-__global__ void __launch_bounds__(kThreads)
-ExpandOwnedWarp(IndexView2 ix, const uint64_t* __restrict__ q_org, uint64_t n_q,
+ExpandOwnedWarp(IndexView ix, const uint64_t* __restrict__ q_org, uint64_t n_q,
                 const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ first,
                 const uint64_t* __restrict__ hit_off, const uint64_t* __restrict__ start,
                 const uint64_t* __restrict__ read_base, uint32_t n_reads, uint32_t parts,
                 uint32_t per_part, uint64_t* __restrict__ h_grp, uint64_t* __restrict__ h_pos,
                 uint32_t* __restrict__ h_lhs, uint32_t* __restrict__ bad) {
-  const uint32_t lane = threadIdx.x & 31;
   const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
-  bool valid = i < n_q;
   uint32_t my_cnt = 0, my_first = 0;
   uint64_t my_org = 0, my_dst = 0;
-  if (valid) {
+  if (i < n_q) {
     my_org = q_org[i];
     const uint32_t lhs_id = static_cast<uint32_t>(my_org >> 32);
     if (lhs_id >= n_reads || i < start[lhs_id] || i >= start[lhs_id + 1]) {
       *bad = 2;  // query records not sorted by read (or a read out of range)
-      valid = false;
     } else {
       my_cnt = cnt[i];
       my_first = first[i];
       my_dst = read_base[Slot(lhs_id, parts, per_part)] + (hit_off[i] - hit_off[start[lhs_id]]);
     }
   }
-  // exclusive prefix of the 32 counts
-  uint32_t incl = my_cnt;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, incl, d);
-    if (lane >= static_cast<uint32_t>(d)) incl += o;
-  }
-  const uint32_t rel = incl - my_cnt;
-  const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
-  for (uint32_t t0 = 0; t0 < total; t0 += 32) {
-    const uint32_t t = t0 + lane;
-    uint32_t q = 0;  // largest q with rel[q] <= t
-#pragma unroll
-    for (uint32_t step = 16; step > 0; step >>= 1) {
-      const uint32_t r = __shfl_sync(0xFFFFFFFFu, rel, q + step);
-      if (r <= t) q += step;
-    }
-    const uint32_t qrel = __shfl_sync(0xFFFFFFFFu, rel, q);
-    const uint32_t qfirst = __shfl_sync(0xFFFFFFFFu, my_first, q);
-    const uint64_t lo = __shfl_sync(0xFFFFFFFFu, my_org, q);
-    const uint64_t qdst = __shfl_sync(0xFFFFFFFFu, my_dst, q);
-    if (t < total) {
-      const uint64_t o = ix.org[qfirst + (t - qrel)];
-      const uint64_t lhs_pos = static_cast<uint32_t>(lo) >> 1;
-      const uint64_t rhs_id = o >> 32;
-      const uint64_t strand = (lo & 1) == (o & 1);
-      const uint64_t rhs_pos = static_cast<uint32_t>(o) >> 1;
-      const uint64_t diagonal =
-          !strand ? rhs_pos + lhs_pos : rhs_pos - lhs_pos + (3ULL << 30);
-      const uint64_t dst = qdst + (t - qrel);
-      h_grp[dst] = (((rhs_id << 1) | strand) << 32) | diagonal;
-      h_pos[dst] = (lhs_pos << 32) | rhs_pos;
-      h_lhs[dst] = static_cast<uint32_t>(lo >> 32);
-    }
-  }
+  __builtin_assume(h_lhs != nullptr);  // (see ExpandOwned)
+  ExpandWarp(ix.org, my_cnt, my_first, my_org, my_dst, h_grp, h_pos, h_lhs);
 }
 
 // ---------------------------------------------------------------------------
@@ -576,8 +439,7 @@ void DistHitsSplit(Ctx& c, const uint64_t* d_qval, const uint64_t* d_qorg, uint6
   if (!c.i_valid) throw StateError("no index");
   CheckParts(parts, 0);
   if (n_query > c.n_reads) throw InvalidArgument("query range out of bounds");
-  IndexView2 ix{ValView{c.i_val.get(), c.i_is32 ? 1 : 0}, c.i_org.get(), c.i_bucket.get(), c.i_n,
-                c.i_shift, c.occurrence, c.i_limit};
+  const IndexView ix = IndexViewOf(c);
   const uint32_t per_part = CeilDiv(n_query, parts);
   const uint64_t slots = static_cast<uint64_t>(per_part) * parts;
   uint32_t* cnt = c.m_cnt.reserve(n_q + 1);
@@ -591,18 +453,7 @@ void DistHitsSplit(Ctx& c, const uint64_t* d_qval, const uint64_t* d_qorg, uint6
   RVN_CUDA(cudaMemsetAsync(bad, 0, 4, c.stream));
   RVN_CUDA(cudaMemsetAsync(tot, 0, (slots + 1) * 4, c.stream));
   TimerBegin(c, "probe");
-  const bool suffix = ae && as && c.i_sorted_ids;  // kept postings = a suffix of the run
-  if (n_q) {
-    if (suffix) {
-      ProbeOwnedSuffix<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(ix, d_qval, d_qorg, n_q,
-                                                                         cnt, frst);
-    } else {
-      ProbeOwned<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(ix, d_qval, d_qorg, n_q, ae,
-                                                                   as, cnt, frst);
-    }
-    RVN_LAUNCH_CHECK();
-    ++c.launches;
-  }
+  ProbeQueries(c, ValView{d_qval, 0}, d_qorg, 0, n_q, ae, as, cnt, frst, nullptr);
   ExclusiveScanU32(c, cnt, off, n_q);
   TimerEnd(c);
   TimerBegin(c, "expand");
@@ -624,7 +475,7 @@ void DistHitsSplit(Ctx& c, const uint64_t* d_qval, const uint64_t* d_qorg, uint6
   uint64_t* hp = c.h_pos.reserve(n_hits + 1);
   uint32_t* hl = c.ds_hit_lhs.reserve(n_hits + 1);
   if (n_q) {
-    if (suffix) {
+    if (KeptContiguous(c, ae, as)) {
       ExpandOwnedWarp<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
           ix, d_qorg, n_q, cnt, frst, off, start, rbase, n_query, parts, per_part, hg, hp, hl, bad);
     } else {

@@ -283,6 +283,13 @@ void MapRange(Ctx& c, uint32_t first, uint32_t last, bool avoid_equal,
               bool avoid_symmetric, bool minhash, bool want_filtered,
               bool fetch = true);
 
+// seed lookup of the queries [q_begin, q_begin + n_q) in their own order (seed.cuh): per
+// query the kept count and the first posting; the over-threshold flags go to filt
+// unless it is null
+void ProbeQueries(Ctx& c, ValView q_val, const uint64_t* q_org, uint64_t q_begin, uint64_t n_q,
+                  bool avoid_equal, bool avoid_symmetric, uint32_t* cnt, uint32_t* first,
+                  uint8_t* filt);
+
 // chains hits grouped by query read (see map.cu); overlaps land in c.m_ovl
 // lhs_ids[i] = id of query read i of the batch (device)
 uint64_t ChainGroupedHits(Ctx& c, const uint64_t* hg, const uint64_t* hp,

@@ -4,10 +4,7 @@
 // RavenLib/src/construct.cc:59-64 -> Map(seq,1,1,1) and :377-381 ->
 // Map(seq,1,1,0,&filtered); algorithm SURVEY.md App. A.2).
 //
-//   probe   one thread per query minimizer: bucket table -> sorted run ->
-//           (first posting, count) or "filtered" if count > occurrence
-//   expand  hits (ram "Match": group = (rhs_id<<1|same_strand)<<32|diagonal,
-//           positions = lhs_pos<<32|rhs_pos) written per query read
+//   probe, expand   see seed.cuh
 //   chain   ONE CTA PER QUERY READ, hits resident in shared memory:
 //           bitonic sort by (group, positions) -> diagonal-band intervals by
 //           binary searches + block scans -> second sort by (band, positions)
@@ -24,69 +21,13 @@
 #include <algorithm>
 
 #include "engine.cuh"
+#include "seed.cuh"
 
 namespace rvn {
 
 namespace {
 
 constexpr int kThreads = 256;
-
-struct IndexView {
-  ValView val;  // sorted values, u32 or u64
-  const uint64_t* org;
-  const uint32_t* bucket;
-  uint64_t n;
-  int shift;
-  uint32_t occurrence;
-  uint64_t limit;  // values beyond it are not indexed (tiered build)
-};
-
-// first record with value v and the run length capped at occurrence+1
-__device__ __forceinline__ void Lookup(const IndexView& ix, uint64_t v,
-                                       uint32_t* first, uint32_t* count) {
-  if (v > ix.limit) {
-    *first = 0;
-    *count = 0;
-    return;
-  }
-  const uint64_t b = v >> ix.shift;
-  uint32_t lo = ix.bucket[b], hi = ix.bucket[b + 1];
-  while (hi - lo > 8) {  // long buckets: bisect down to a short scan
-    const uint32_t mid = lo + (hi - lo) / 2;
-    if (ix.val[mid] < v) {
-      lo = mid + 1;
-    } else {
-      hi = mid;
-    }
-  }
-  // here every record before lo is < v; the run (if any) starts in [lo, hi]
-  const uint32_t end = ix.bucket[b + 1];
-  while (lo < end && ix.val[lo] < v) ++lo;
-  if (lo >= end || ix.val[lo] != v) {
-    *first = 0;
-    *count = 0;
-    return;
-  }
-  *first = lo;
-  if (ix.occurrence != 0xFFFFFFFFu &&
-      static_cast<uint64_t>(lo) + ix.occurrence < ix.n &&
-      ix.val[static_cast<uint64_t>(lo) + ix.occurrence] == v) {
-    *count = ix.occurrence + 1;  // over the threshold, exact length not needed
-    return;
-  }
-  uint32_t n = 1;
-  while (static_cast<uint64_t>(lo) + n < ix.n && ix.val[lo + n] == v) ++n;
-  *count = n;
-}
-
-__device__ __forceinline__ bool KeepPosting(uint32_t lhs_id, uint64_t origin,
-                                            bool avoid_equal,
-                                            bool avoid_symmetric) {
-  const uint32_t rhs_id = static_cast<uint32_t>(origin >> 32);
-  if (avoid_equal && lhs_id == rhs_id) return false;
-  if (avoid_symmetric && lhs_id > rhs_id) return false;
-  return true;
-}
 
 __global__ void __launch_bounds__(kThreads)
 ProbeKernel(IndexView ix, ValView q_val,
@@ -96,23 +37,12 @@ ProbeKernel(IndexView ix, ValView q_val,
             uint8_t* __restrict__ filt) {
   const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
   if (i >= n_q) return;
-  const uint64_t v = q_val[q_begin + i];
-  const uint32_t lhs_id = static_cast<uint32_t>(q_org[q_begin + i] >> 32);
-  uint32_t f, n;
-  Lookup(ix, v, &f, &n);
-  uint32_t kept = 0;
-  uint8_t over = 0;
-  if (n > ix.occurrence) {
-    over = 1;
-    n = 0;
-  } else {
-    for (uint32_t j = 0; j < n; ++j) {
-      kept += KeepPosting(lhs_id, ix.org[f + j], avoid_equal, avoid_symmetric);
-    }
-  }
+  uint32_t f, kept;
+  const bool over = Probe(ix, q_val[q_begin + i], [&] { return static_cast<uint32_t>(q_org[q_begin + i] >> 32); },
+                          Kept::kFiltered, avoid_equal, avoid_symmetric, &f, &kept);
   cnt[i] = kept;
   first[i] = f;
-  filt[i] = over;
+  if (filt) filt[i] = over;
   // the posting count is re-derived in ExpandKernel from the run itself
 }
 
@@ -126,36 +56,14 @@ ExpandKernel(IndexView ix, ValView q_val,
              uint64_t* __restrict__ h_pos) {
   const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
   if (i >= n_q) return;
-  uint32_t left = cnt[i];
+  const uint32_t left = cnt[i];
   if (left == 0) return;
-  const uint64_t v = q_val[q_begin + i];
-  const uint64_t lo = q_org[q_begin + i];
-  const uint32_t lhs_id = static_cast<uint32_t>(lo >> 32);
-  const uint64_t lhs_pos = static_cast<uint32_t>(lo) >> 1;
-  uint64_t dst = hit_off[i];
-  for (uint64_t j = first[i]; left > 0 && j < ix.n && ix.val[j] == v; ++j) {
-    const uint64_t o = ix.org[j];
-    if (!KeepPosting(lhs_id, o, avoid_equal, avoid_symmetric)) continue;
-    const uint64_t rhs_id = o >> 32;
-    const uint64_t strand = (lo & 1) == (o & 1);
-    const uint64_t rhs_pos = static_cast<uint32_t>(o) >> 1;
-    const uint64_t diagonal =
-        !strand ? rhs_pos + lhs_pos : rhs_pos - lhs_pos + (3ULL << 30);
-    h_grp[dst] = (((rhs_id << 1) | strand) << 32) | diagonal;
-    h_pos[dst] = (lhs_pos << 32) | rhs_pos;
-    ++dst;
-    --left;
-  }
+  ExpandQuery(ix, q_val[q_begin + i], q_org[q_begin + i], first[i], left, avoid_equal,
+              avoid_symmetric, hit_off[i], h_grp, h_pos, nullptr);
 }
 
-// ---- fast path of probe + expand -------------------------------------------
-// The postings of a key are in read order (the index sort is stable over
-// records in (read, position) order), so with avoid_equal && avoid_symmetric
-// the kept postings (rhs_id > lhs_id) are a SUFFIX of the run - and with both
-// flags off they are the whole run. The probe then only needs the first kept
-// posting (a binary search in the run), and the expansion can be done by whole
-// warps with fully coalesced stores: hit t of a warp's 32 queries is located
-// by a shuffle search over the 32 exclusive prefixes.
+// ---- fast path of probe + expand: the kept postings are contiguous ----
+// strict_above: they are the suffix rhs_id > lhs_id, else the whole run
 __global__ void __launch_bounds__(kThreads)
 ProbeSuffixKernel(IndexView ix, ValView q_val,
                   const uint64_t* __restrict__ q_org, uint64_t q_begin, uint64_t n_q,
@@ -163,28 +71,12 @@ ProbeSuffixKernel(IndexView ix, ValView q_val,
                   uint32_t* __restrict__ first, uint8_t* __restrict__ filt) {
   const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
   if (i >= n_q) return;
-  const uint64_t v = q_val[q_begin + i];
-  uint32_t f, n;
-  Lookup(ix, v, &f, &n);
-  uint8_t over = 0;
-  uint32_t kept = 0, fk = f;
-  if (n > ix.occurrence) {
-    over = 1;
-  } else if (n > 0) {
-    if (strict_above) {
-      const uint32_t lhs_id = static_cast<uint32_t>(q_org[q_begin + i] >> 32);
-      uint32_t lo = f, hi = f + n;  // first posting with rhs_id > lhs_id
-      while (lo < hi) {
-        const uint32_t mid = lo + (hi - lo) / 2;
-        if (static_cast<uint32_t>(ix.org[mid] >> 32) <= lhs_id) lo = mid + 1; else hi = mid;
-      }
-      fk = lo;
-    }
-    kept = f + n - fk;
-  }
+  uint32_t fk, kept;
+  const bool over = Probe(ix, q_val[q_begin + i], [&] { return static_cast<uint32_t>(q_org[q_begin + i] >> 32); },
+                          strict_above ? Kept::kSuffix : Kept::kWholeRun, true, true, &fk, &kept);
   cnt[i] = kept;
   first[i] = fk;
-  filt[i] = over;
+  if (filt) filt[i] = over;
 }
 
 // the same probe over queries sorted by value: neighbouring threads walk
@@ -197,26 +89,10 @@ ProbeSortedKernel(IndexView ix, ValView sorted_val,
                   bool strict_above, uint64_t* __restrict__ packed) {
   const uint64_t t = static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x;
   if (t >= n_q) return;
-  const uint64_t v = sorted_val[t];
   const uint32_t i = sorted_idx[t];
-  uint32_t f, n;
-  Lookup(ix, v, &f, &n);
-  uint8_t over = 0;
-  uint32_t kept = 0, fk = f;
-  if (n > ix.occurrence) {
-    over = 1;
-  } else if (n > 0) {
-    if (strict_above) {
-      const uint32_t lhs_id = static_cast<uint32_t>(q_org[q_begin + i] >> 32);
-      uint32_t lo = f, hi = f + n;
-      while (lo < hi) {
-        const uint32_t mid = lo + (hi - lo) / 2;
-        if (static_cast<uint32_t>(ix.org[mid] >> 32) <= lhs_id) lo = mid + 1; else hi = mid;
-      }
-      fk = lo;
-    }
-    kept = f + n - fk;
-  }
+  uint32_t fk, kept;
+  const bool over = Probe(ix, sorted_val[t], [&] { return static_cast<uint32_t>(q_org[q_begin + i] >> 32); },
+                          strict_above ? Kept::kSuffix : Kept::kWholeRun, true, true, &fk, &kept);
   // ONE scattered store per query (a partial-sector write costs a read-modify-
   // write in HBM): first kept posting | over-threshold flag | kept count
   packed[i] = (static_cast<uint64_t>(fk) << 32) | (static_cast<uint64_t>(over) << 31) | kept;
@@ -239,49 +115,10 @@ ExpandWarpKernel(IndexView ix, const uint64_t* __restrict__ q_org, uint64_t q_be
                  uint64_t n_q, const uint32_t* __restrict__ cnt,
                  const uint32_t* __restrict__ first, const uint64_t* __restrict__ hit_off,
                  uint64_t* __restrict__ h_grp, uint64_t* __restrict__ h_pos) {
-  const uint32_t lane = threadIdx.x & 31;
   const uint64_t i = (static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x);
   const bool valid = i < n_q;
-  const uint32_t my_cnt = valid ? cnt[i] : 0;
-  const uint32_t my_first = valid ? first[i] : 0;
-  const uint64_t my_org = valid ? q_org[q_begin + i] : 0;
-  const uint64_t my_off = valid ? hit_off[i] : 0;
-  // exclusive prefix of the warp, relative to its first query (lanes beyond n_q
-  // only occur at the very end: give them the running end)
-  const uint64_t base = __shfl_sync(0xFFFFFFFFu, my_off, 0);
-  uint32_t rel = valid ? static_cast<uint32_t>(my_off - base) : 0;
-  // total and a monotone prefix for the invalid tail lanes
-  uint32_t run = valid ? rel + my_cnt : 0;
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, run, d);
-    if (lane >= d && o > run) run = o;
-  }
-  if (!valid) rel = run;
-  const uint32_t total = __shfl_sync(0xFFFFFFFFu, run, 31);
-  for (uint32_t t0 = 0; t0 < total; t0 += 32) {
-    const uint32_t t = t0 + lane;
-    // largest q with rel[q] <= t
-    uint32_t q = 0;
-#pragma unroll
-    for (uint32_t step = 16; step > 0; step >>= 1) {
-      const uint32_t r = __shfl_sync(0xFFFFFFFFu, rel, q + step);
-      if (r <= t) q += step;
-    }
-    const uint32_t qrel = __shfl_sync(0xFFFFFFFFu, rel, q);
-    const uint32_t qfirst = __shfl_sync(0xFFFFFFFFu, my_first, q);
-    const uint64_t lo = __shfl_sync(0xFFFFFFFFu, my_org, q);
-    if (t < total) {
-      const uint64_t o = ix.org[qfirst + (t - qrel)];
-      const uint64_t lhs_pos = static_cast<uint32_t>(lo) >> 1;
-      const uint64_t rhs_id = o >> 32;
-      const uint64_t strand = (lo & 1) == (o & 1);
-      const uint64_t rhs_pos = static_cast<uint32_t>(o) >> 1;
-      const uint64_t diagonal =
-          !strand ? rhs_pos + lhs_pos : rhs_pos - lhs_pos + (3ULL << 30);
-      h_grp[base + t] = (((rhs_id << 1) | strand) << 32) | diagonal;
-      h_pos[base + t] = (lhs_pos << 32) | rhs_pos;
-    }
-  }
+  ExpandWarp(ix.org, valid ? cnt[i] : 0, valid ? first[i] : 0, valid ? q_org[q_begin + i] : 0,
+             valid ? hit_off[i] : 0, h_grp, h_pos, nullptr);
 }
 
 // ---- stage-1 hits by a self-join over the index ----
@@ -362,7 +199,6 @@ __global__ void __launch_bounds__(kThreads)
 ExpandJoinKernel(const uint64_t* __restrict__ i_org, const uint64_t* __restrict__ packed,
                  uint64_t n_q, const uint64_t* __restrict__ hit_off,
                  uint64_t* __restrict__ h_grp, uint64_t* __restrict__ h_pos) {
-  const uint32_t lane = threadIdx.x & 31;
   const uint64_t i = (static_cast<uint64_t>(blockIdx.x) * kThreads + threadIdx.x);
   const bool valid = i < n_q;
   const uint64_t pk = valid ? packed[i] : 0;
@@ -375,39 +211,7 @@ ExpandJoinKernel(const uint64_t* __restrict__ i_org, const uint64_t* __restrict_
     my_first = post + 1;
     while ((i_org[my_first] >> 32) == (my_org >> 32)) ++my_first;  // same read: not a hit
   }
-  const uint64_t my_off = valid ? hit_off[i] : 0;
-  const uint64_t base = __shfl_sync(0xFFFFFFFFu, my_off, 0);
-  uint32_t rel = valid ? static_cast<uint32_t>(my_off - base) : 0;
-  uint32_t run = valid ? rel + my_cnt : 0;
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, run, d);
-    if (lane >= d && o > run) run = o;
-  }
-  if (!valid) rel = run;
-  const uint32_t total = __shfl_sync(0xFFFFFFFFu, run, 31);
-  for (uint32_t t0 = 0; t0 < total; t0 += 32) {
-    const uint32_t t = t0 + lane;
-    uint32_t q = 0;
-#pragma unroll
-    for (uint32_t step = 16; step > 0; step >>= 1) {
-      const uint32_t r = __shfl_sync(0xFFFFFFFFu, rel, q + step);
-      if (r <= t) q += step;
-    }
-    const uint32_t qrel = __shfl_sync(0xFFFFFFFFu, rel, q);
-    const uint32_t qfirst = __shfl_sync(0xFFFFFFFFu, my_first, q);
-    const uint64_t lo = __shfl_sync(0xFFFFFFFFu, my_org, q);
-    if (t < total) {
-      const uint64_t o = i_org[qfirst + (t - qrel)];
-      const uint64_t lhs_pos = static_cast<uint32_t>(lo) >> 1;
-      const uint64_t rhs_id = o >> 32;
-      const uint64_t strand = (lo & 1) == (o & 1);
-      const uint64_t rhs_pos = static_cast<uint32_t>(o) >> 1;
-      const uint64_t diagonal =
-          !strand ? rhs_pos + lhs_pos : rhs_pos - lhs_pos + (3ULL << 30);
-      h_grp[base + t] = (((rhs_id << 1) | strand) << 32) | diagonal;
-      h_pos[base + t] = (lhs_pos << 32) | rhs_pos;
-    }
-  }
+  ExpandWarp(i_org, my_cnt, my_first, my_org, valid ? hit_off[i] : 0, h_grp, h_pos, nullptr);
 }
 
 // per-read offsets out of per-record offsets
@@ -1614,6 +1418,22 @@ uint64_t ChainGroupedHits(Ctx& c, const uint64_t* hg, const uint64_t* hp,
   return n_ovl;
 }
 
+void ProbeQueries(Ctx& c, ValView q_val, const uint64_t* q_org, uint64_t q_begin, uint64_t n_q,
+                  bool avoid_equal, bool avoid_symmetric, uint32_t* cnt, uint32_t* first,
+                  uint8_t* filt) {
+  if (n_q == 0) return;
+  const IndexView ix = IndexViewOf(c);
+  if (KeptContiguous(c, avoid_equal, avoid_symmetric)) {
+    ProbeSuffixKernel<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
+        ix, q_val, q_org, q_begin, n_q, avoid_equal, cnt, first, filt);
+  } else {
+    ProbeKernel<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
+        ix, q_val, q_org, q_begin, n_q, avoid_equal, avoid_symmetric, cnt, first, filt);
+  }
+  RVN_LAUNCH_CHECK();
+  ++c.launches;
+}
+
 void MapRange(Ctx& c, uint32_t first, uint32_t last, bool avoid_equal,
               bool avoid_symmetric, bool minhash, bool want_filtered,
               bool fetch) {
@@ -1706,8 +1526,7 @@ void MapRange(Ctx& c, uint32_t first, uint32_t last, bool avoid_equal,
   const uint64_t q_begin = (*h_read_off)[off_base_read];
   n_q = (*h_read_off)[off_base_read + nr] - q_begin;
 
-  IndexView ix{ValView{c.i_val.get(), c.i_is32 ? 1 : 0}, c.i_org.get(), c.i_bucket.get(), c.i_n,
-               c.i_shift, c.occurrence, c.i_limit};
+  const IndexView ix = IndexViewOf(c);
 
   // ---- probe + expand ----
   TimerBegin(c, "probe");
@@ -1715,9 +1534,7 @@ void MapRange(Ctx& c, uint32_t first, uint32_t last, bool avoid_equal,
   uint32_t* frst = c.m_first.reserve(n_q + 1);
   uint8_t* filt = c.m_filt.reserve(n_q + 1);
   uint64_t* hit_off = c.m_hit_off.reserve(n_q + 2);
-  // kept postings = a suffix of the run (or the whole run): see ProbeSuffixKernel
-  const bool suffix = (avoid_equal && avoid_symmetric && c.i_sorted_ids) ||
-                      (!avoid_equal && !avoid_symmetric);
+  const bool suffix = KeptContiguous(c, avoid_equal, avoid_symmetric);
   if (n_q > 0) {
     if (suffix && n_q >= (1u << 16) && n_q < 0xFFFFFFFFULL) {
       // sort the queries by value, probe in that order, results back by index
@@ -1749,16 +1566,11 @@ void MapRange(Ctx& c, uint32_t first, uint32_t last, bool avoid_equal,
       ProbeSortedKernel<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
           ix, sorted_qv, sorted_qi, qo, q_begin, n_q, avoid_equal, packed);
       UnpackProbe<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(packed, n_q, cnt, frst, filt);
-      c.launches += (2 * c.prm.k + 7) / 8 + 5;
-    } else if (suffix) {
-      ProbeSuffixKernel<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
-          ix, qv, qo, q_begin, n_q, avoid_equal, cnt, frst, filt);
+      RVN_LAUNCH_CHECK();
+      c.launches += (2 * c.prm.k + 7) / 8 + 6;
     } else {
-      ProbeKernel<<<CeilDiv(n_q, kThreads), kThreads, 0, c.stream>>>(
-          ix, qv, qo, q_begin, n_q, avoid_equal, avoid_symmetric, cnt, frst, filt);
+      ProbeQueries(c, qv, qo, q_begin, n_q, avoid_equal, avoid_symmetric, cnt, frst, filt);
     }
-    RVN_LAUNCH_CHECK();
-    ++c.launches;
     ExclusiveScanU32(c, cnt, hit_off, n_q);
     n_hits = ReadU64(c, hit_off + n_q);
   } else {
